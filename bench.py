@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the contract benchmark of the OneSweep path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE pass of the hot path over one batch of synthetic input: one OneSweep sort of 2^30 uint32 keys
@@ -73,6 +73,7 @@ def workload(log2n: int, world: int) -> str:
 SEED = 10              # the reference's benchmark seed (GPUSortingCUDA.cu:22)
 CPU_SAMPLE_LOG2 = 27   # bounded CPU sample of the same workload (1/8 of it)
 ALG_BYTES_PER_KEY_PER_PASS = 8  # SURVEY 8(d): one DigitBinningPass reads 4 B and writes 4 B per key
+DUMP_SAMPLE = 1 << 22  # --dump-outputs: values kept per output array
 
 
 def measured_peak_gbs():
@@ -151,7 +152,8 @@ class ClockSampler(threading.Thread):
 
 def _cpu_sort_sample(steps: int, warmup: int):
     """The CPU leg shared by cpu_baseline and --impl reference: the oracle's host-parallel OneSweep port on
-    HOST_THREADS threads over a 2^CPU_SAMPLE_LOG2-key sample of the workload.  Returns (best_s, mean_s, all_s, orc, src)."""
+    HOST_THREADS threads over a 2^CPU_SAMPLE_LOG2-key sample of the workload.  Returns (best_s, mean_s, all_s, orc, src, work),
+    work holding the last timed step's sorted keys."""
     from tests import oraclelib
     import numpy as np
 
@@ -170,7 +172,7 @@ def _cpu_sort_sample(steps: int, warmup: int):
         orc.sort_parallel_inplace(work, threads=HOST_THREADS, alt=alt)
         times.append(time.perf_counter() - t0)
     assert orc.validate(work) == 0
-    return min(times), sum(times) / len(times), times, orc, src
+    return min(times), sum(times) / len(times), times, orc, src, work
 
 
 def _sample_text(kind: str) -> str:
@@ -183,7 +185,7 @@ def cpu_baseline():
     """Bounded CPU sample: the oracle's host-parallel OneSweep port on all physical cores + std::sort on one core."""
     import numpy as np
 
-    best, mean, times, orc, src = _cpu_sort_sample(steps=5, warmup=1)
+    best, mean, times, orc, src, _ = _cpu_sort_sample(steps=5, warmup=1)
     n = src.size
     m = 1 << 24
     w2 = src[:m].copy()
@@ -210,7 +212,12 @@ def run_reference_arm(args, rank, world, emit):
     CPU side; the mean is reported beside it)."""
     if rank != 0:
         return
-    best, mean, times, orc, src = _cpu_sort_sample(steps=args.steps, warmup=args.warmup)
+    best, mean, times, orc, src, work = _cpu_sort_sample(steps=args.steps, warmup=args.warmup)
+    if args.dump_outputs:
+        import numpy as np
+        import torch
+
+        dump_outputs(args.dump_outputs, {"sorted_keys": torch.from_numpy(work.view(np.int32))})
     n = src.size
     value = n / best / 1e9
     line = {
@@ -247,7 +254,14 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip extra_configs (pairs, u64) and ref_cuda (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the sorted keys of the last one to DIR/sorted_keys.npy (float64; "
+                         f"a fixed seeded sample of {DUMP_SAMPLE} positions when the output is larger), so that two builds "
+                         "can be compared output for output.  With N > 1 GPUs every rank writes its slice of the global "
+                         f"order to DIR/sorted_keys_rank<r>.npy, sampled to {DUMP_SAMPLE} / N positions")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "ours" and args.warmup < 3:
         print(f"bench.py: --warmup {args.warmup} raised to 3 (timing rule: W >= 3)", file=sys.stderr)
         args.warmup = 3
@@ -361,6 +375,23 @@ def multiset_checksum(t):
         b += int(((x * 2654435761) ^ (x >> 7)).sum().item())
     m = (1 << 64) - 1
     return a & m, b & m
+
+
+def dump_outputs(out_dir, arrays, sample=DUMP_SAMPLE):
+    """Writes each tensor of 32-bit unsigned words as out_dir/<name>.npy in float64 (exact for 32-bit values).  A tensor
+    longer than `sample` is sampled at `sample` distinct positions drawn with seed SEED and kept in ascending order, the
+    same positions on every run with the same arguments; DUMP_SAMPLE float64 values are 32 MiB."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        if flat.numel() > sample:
+            idx = np.sort(np.random.default_rng(SEED).choice(flat.numel(), size=sample, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        vals = flat.to(torch.int64).cpu().numpy() & 0xFFFFFFFF
+        np.save(os.path.join(out_dir, f"{name}.npy"), vals.astype(np.float64))
 
 
 def _time_sorts(steps, warmup, restore, sort, stream):
@@ -521,6 +552,9 @@ def bench_single(args, g, n, device_index):
     for _ in range(args.warmup):
         one_step(False)
     torch.cuda.synchronize()
+    # the handle's pass counter advances once per digit place of every multi-kernel sort (4 for uint32 keys), so it counts
+    # the sorts the timed loop really issued (bench sizes are far above the one-launch small-n path, which has no pass)
+    epoch0 = s.info("epoch")
     sampler = ClockSampler(device_index)
     sampler.start()
     events, profiles = [], []
@@ -536,8 +570,11 @@ def bench_single(args, g, n, device_index):
                  "digit_binning_pass_mean": float(prof[:, 2:].mean())}
     for p in range(prof.shape[1] - 2):
         kernel_ms[f"digit_binning_pass_{p}"] = float(prof[:, 2 + p].mean())
+    timed_sorts = (s.info("epoch") - epoch0) // 4
     # sorted (the reference's Validate) AND the same multiset as the input (an output of equal keys would not pass)
     verified = s.validate(work) == 0 and multiset_checksum(work) == checksum_in
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sorted_keys": work})
     launches = s.info("launches_per_sort")
 
     # ---- end to end through the C-ABI host entry point, pinned host memory ---------------------------------
@@ -569,7 +606,7 @@ def bench_single(args, g, n, device_index):
         "kernel": "digit_binning_wide_kernel" if variant == 2 else ("digit_binning_persistent_kernel" if variant == 1 else "digit_binning_tile_kernel"),
         "variant": variant, "tile_keys": tile_keys, "rank_mode": "atomic" if rank_mode == 0 else "ballot",
         "e2e_ms_per_step": e2e_ms, "e2e_steps": e2e_steps, "h2d_bytes": 4 * n, "d2h_bytes": 4 * n,
-        "gpu_launches": args.steps * launches, "clocks": clocks, "verified": verified,
+        "gpu_launches": timed_sorts * launches, "clocks": clocks, "verified": verified,
     }
     if not args.no_extra:
         peak, _ = measured_peak_gbs()

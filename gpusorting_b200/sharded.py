@@ -186,7 +186,7 @@ def bench_sharded(args, rank: int, world: int, local_rank: int, n: int):
     from . import init_random
     from .onesweep import OneSweepSorter  # noqa: F401
 
-    from bench import ClockSampler, SEED  # type: ignore
+    from bench import DUMP_SAMPLE, SEED, ClockSampler, dump_outputs  # type: ignore
 
     src = torch.empty(n, dtype=torch.int32, device="cuda")
     init_random(src, 0, SEED + rank)
@@ -231,6 +231,8 @@ def bench_sharded(args, rank: int, world: int, local_rank: int, n: int):
     dist.all_reduce(total_out)
     verified = (verify_global_order(res, rank, world) and int(total_out) == int(total_in)
                 and global_multiset_checksum(res) == checksum_in)
+    if args.dump_outputs:  # this rank's slice of the global order, as ShardedSorter.sort_keys returned it
+        dump_outputs(args.dump_outputs, {f"sorted_keys_rank{rank}": res}, DUMP_SAMPLE // world)
     ph = {k: float(np.mean([p[k] for p in phases])) for k in phases[0]}
     # every rank's own view (phases are measured by the rank's own CUDA events; a rank that arrives early at a collective
     # waits inside the phase that contains it)

@@ -17,11 +17,3 @@ def oracle():
     from tests import oraclelib
 
     return oraclelib.load_oracle()
-
-
-@pytest.fixture(scope="session")
-def reflib():
-    """The reference's own CUDA kernels (oracle/_ref/libref_onesweep.so), or None if it was not built."""
-    from tests import oraclelib
-
-    return oraclelib.load_ref()

@@ -1,6 +1,6 @@
 """ctypes access to the TEST-ONLY libraries under oracle/ (the CPU restatement and, when built, the
-reference's own CUDA kernels).  Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs may
-import this module; nothing under gpusorting_b200/ does."""
+reference's own CUDA kernels), and the tensor digest the golden fixtures store.  Only tests/, __graft_entry__.smoke()
+and bench.py's CPU-baseline legs may import this module; nothing under gpusorting_b200/ does."""
 from __future__ import annotations
 
 import ctypes
@@ -123,6 +123,25 @@ def load_oracle() -> Oracle:
     if not os.path.exists(ORACLE_SO):
         build_oracle()
     return Oracle(ctypes.CDLL(ORACLE_SO))
+
+
+def device_digest(t) -> int:
+    """Order-sensitive 64-bit checksum of a tensor's 32-bit words, computed where the tensor lives.  Each word is mixed with
+    its index and the mixes are summed with wrapping int64 arithmetic, so the value does not depend on reduction order;
+    moving a word to another index changes it.  Digests of the reference's 2^30-element outputs are stored under
+    tests/golden/, where a host-side hash of 4 GiB per array would take seconds each."""
+    import torch
+
+    flat = t.reshape(-1).view(torch.int32)
+    k1, k2 = 0x2545F4914F6CDD1D, 0x5851F42D4C957F2D
+    h, step = 0, 1 << 26
+    for s in range(0, flat.numel(), step):
+        x = flat[s:s + step].to(torch.int64) & 0xFFFFFFFF
+        i = torch.arange(s, s + x.numel(), dtype=torch.int64, device=x.device)
+        y = (x ^ (i * k1)) * k2
+        y = (y ^ (y >> 29)) * k1
+        h += int(y.sum().item())
+    return h & ((1 << 64) - 1)
 
 
 class RefCuda:

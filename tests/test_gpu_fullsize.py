@@ -1,11 +1,23 @@
 """BASELINE.json's full sizes (2^30) through size-independent properties: sortedness (the reference's Validate),
-conservation of every digit-place histogram, a multiset checksum, stability via payload order, and -- when
-oracle/_ref exists -- bit-exact equality with the reference's CUDA OneSweep.  Needs a B200: -m gpu."""
+conservation of every digit-place histogram, a multiset checksum, stability via payload order, and bit-exact
+equality with the reference's CUDA OneSweep through device digests of its outputs (tests/golden/).  Needs a B200: -m gpu."""
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
 
+from tests.oraclelib import device_digest
+
 pytestmark = pytest.mark.gpu
+
+PARITY_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_onesweep_parity_golden.json")
+
+
+def reference_case(name):
+    """Digests of the input and of the reference CUDA OneSweep's output for one 2^30 case (tests/golden/make_ref_golden.py)."""
+    return json.load(open(PARITY_GOLDEN))["fullsize"][name]
 
 
 def multiset_checksum(t):
@@ -29,28 +41,21 @@ def g():
     return g
 
 
-def test_keys_u32_2pow30(g, reflib):
+def test_keys_u32_2pow30(g):
     n = 1 << 30
+    ref = reference_case("keys_u32")  # the reference is valid up to exactly 2^30 (30-bit descriptor value, SURVEY D5)
+    assert ref["n"] == n
     s = g.OneSweepSorter(n, 4, 0)
     t = torch.empty(n, dtype=torch.int32, device="cuda")
-    g.init_random(t, 0, 10)
+    g.init_random(t, 0, ref["seed"])
+    assert device_digest(t) == ref["input_digest"]
     h0 = s.global_histogram(t).clone()
     c0 = multiset_checksum(t)
-    ref_out = None
-    if reflib is not None:  # the reference is valid up to exactly 2^30 (30-bit descriptor value, SURVEY D5)
-        h = reflib.lib.ref_create(n)
-        a, alt = t.clone(), torch.empty_like(t)
-        assert reflib.lib.ref_sort_keys(h, a.data_ptr(), alt.data_ptr(), n) == 0
-        torch.cuda.synchronize()
-        del alt
-        ref_out = a
-        reflib.lib.ref_destroy(h)
     s.sort_keys(t)
     assert s.validate(t) == 0
     assert torch.equal(s.global_histogram(t), h0)
     assert multiset_checksum(t) == c0
-    if ref_out is not None:
-        assert torch.equal(t, ref_out)
+    assert device_digest(t) == ref["sorted_digest"], "keys differ from the reference CUDA OneSweep"
     # idempotence: sorting sorted data changes nothing
     first = t[: 1 << 20].clone()
     s.sort_keys(t)
@@ -79,44 +84,30 @@ def test_pairs_u32_2pow30_stability(g):
     s.close()
 
 
-def test_pairs_u32_2pow30_bit_exact_vs_reference_cuda(g, reflib):
+def test_pairs_u32_2pow30_bit_exact_vs_reference_cuda(g):
     """BASELINE config 3 as SURVEY 8(d) states it: 2^30 (key, payload) pairs, keys AND payloads bit-exact against the
     reference's own pairs kernels (OneSweep::DigitBinningPassPairs, Sort/OneSweep.cu:346-600) on identical input.
     Payload = element index and 20-bit keys (~1024 duplicates of every key value): any instability in either
     implementation would show as a payload mismatch."""
-    if reflib is None:
-        pytest.skip("oracle/_ref/libref_onesweep.so not built")
     n = 1 << 30
+    ref = reference_case("pairs_u32_index_payload")
+    assert ref["n"] == n
     k = torch.empty(n, dtype=torch.int32, device="cuda")
     v = torch.empty(n, dtype=torch.int32, device="cuda")
-    g.init_random(k, 0, 10, payload=v, payload_is_index=True)
-    k &= 0xFFFFF
-    rk, rv = k.clone(), v.clone()
-    h = reflib.lib.ref_create(n)
-    assert h
-    ak, av = torch.empty_like(k), torch.empty_like(v)
-    assert reflib.lib.ref_sort_pairs(h, rk.data_ptr(), rv.data_ptr(), ak.data_ptr(), av.data_ptr(), n) == 0
-    torch.cuda.synchronize()
-    del ak, av
-    reflib.lib.ref_destroy(h)
-    torch.cuda.empty_cache()
+    g.init_random(k, 0, ref["seed"], payload=v, payload_is_index=True)
+    k &= ref["key_mask"]
+    assert device_digest(k) == ref["input_digest"] and device_digest(v) == ref["input_payload_digest"]
     s = g.OneSweepSorter(n, 4, 4)
     s.sort_pairs(k, v)
-    torch.cuda.synchronize()
-    assert torch.equal(k, rk), "keys differ from the reference CUDA OneSweep"
-    assert torch.equal(v, rv), "payloads differ from the reference CUDA OneSweep"
+    assert device_digest(k) == ref["sorted_digest"], "keys differ from the reference CUDA OneSweep"
+    assert device_digest(v) == ref["payload_digest"], "payloads differ from the reference CUDA OneSweep"
     # and with the reference's own payload = key input (UtilityKernels.cuh:85-117), full 32-bit keys
-    g.init_random(k, 0, 10, payload=v)
-    rk.copy_(k); rv.copy_(v)
+    ref = reference_case("pairs_u32_key_payload")
+    g.init_random(k, 0, ref["seed"], payload=v)
+    assert device_digest(k) == ref["input_digest"] and device_digest(v) == ref["input_payload_digest"]
     s.sort_pairs(k, v)
     s.close()
-    torch.cuda.empty_cache()
-    h = reflib.lib.ref_create(n)
-    ak, av = torch.empty_like(k), torch.empty_like(v)
-    assert reflib.lib.ref_sort_pairs(h, rk.data_ptr(), rv.data_ptr(), ak.data_ptr(), av.data_ptr(), n) == 0
-    torch.cuda.synchronize()
-    reflib.lib.ref_destroy(h)
-    assert torch.equal(k, rk) and torch.equal(v, rv)
+    assert device_digest(k) == ref["sorted_digest"] and device_digest(v) == ref["payload_digest"]
 
 
 def test_keys_u64_2pow30(g):

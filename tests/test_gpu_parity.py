@@ -1,5 +1,5 @@
-"""Parity of the CUDA path (through the C-ABI) with the oracle, bit-exact, on seeded inputs -- plus, when
-oracle/_ref was built, with the reference's own CUDA kernels on identical inputs.  Needs a B200: -m gpu."""
+"""Parity of the CUDA path (through the C-ABI) with the oracle, bit-exact, on seeded inputs -- plus with the
+reference's own CUDA kernels on identical inputs, through the fixtures they produced (tests/golden/).  Needs a B200: -m gpu."""
 import json
 import os
 
@@ -7,11 +7,14 @@ import numpy as np
 import pytest
 import torch
 
+from tests.oraclelib import device_digest
+
 pytestmark = pytest.mark.gpu
 
 DEFAULT_VARIANT = 2
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_onesweep_golden.json")
+PARITY_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_onesweep_parity_golden.json")
 
 
 def dev_u32(a):
@@ -42,29 +45,26 @@ def tile_keys(sorter):
 
 # ---- against the reference's own CUDA kernels ------------------------------------------------------
 
-def test_bit_exact_vs_reference_cuda(g, sorter, reflib):
-    if reflib is None:
-        pytest.skip("oracle/_ref/libref_onesweep.so not built")
+def test_bit_exact_vs_reference_cuda(g, sorter):
+    """Keys and pairs (payload = key, as the reference generates them) against the reference's CUDA OneSweep on the
+    same inputs, through device digests of its inputs and outputs (tests/golden/make_ref_golden.py)."""
+    cases = json.load(open(PARITY_GOLDEN))["bit_exact"]
+    assert [(c["n"], c["seed"]) for c in cases] == [(7680, 7680), (9999, 9999), (1 << 20, 10), (1 << 22, 22)]
     n = 1 << 22
-    h = reflib.lib.ref_create(n)
-    a, alt = torch.empty(n, dtype=torch.int32, device="cuda"), torch.empty(n, dtype=torch.int32, device="cuda")
-    pa, palt = torch.empty_like(a), torch.empty_like(a)
-    for size, seed in [(7680, 7680), (9999, 9999), (1 << 20, 10), (1 << 22, 22)]:
-        assert reflib.lib.ref_init_random_keys(a.data_ptr(), size, 0, seed) == 0
-        mine = a[:size].clone()
-        assert reflib.lib.ref_sort_keys(h, a.data_ptr(), alt.data_ptr(), size) == 0
+    a, pa = torch.empty(n, dtype=torch.int32, device="cuda"), torch.empty(n, dtype=torch.int32, device="cuda")
+    for c in cases:
+        size, want = c["n"], c["keys"]
+        mine = a[:size]
+        g.init_random(mine, 0, c["seed"])
+        assert device_digest(mine) == want["input_digest"], f"keys input n={size}"
         sorter.sort_keys(mine)
-        torch.cuda.synchronize()
-        assert torch.equal(mine, a[:size]), f"keys n={size}"
-        # pairs, payload = key as the reference generates them
-        assert reflib.lib.ref_init_random_pairs(a.data_ptr(), pa.data_ptr(), size, 0, seed) == 0
-        mk, mv = a[:size].clone(), pa[:size].clone()
-        assert reflib.lib.ref_sort_pairs(h, a.data_ptr(), pa.data_ptr(), alt.data_ptr(), palt.data_ptr(), size) == 0
+        assert device_digest(mine) == want["sorted_digest"], f"keys n={size}"
+        assert want["ref_validate_errors"] == 0 and sorter.validate(mine) == 0
+        mk, mv, want = a[:size], pa[:size], c["pairs"]
+        g.init_random(mk, 0, c["seed"], payload=mv)
+        assert device_digest(mk) == want["input_digest"] and device_digest(mv) == want["input_payload_digest"], f"pairs input n={size}"
         sorter.sort_pairs(mk, mv)
-        torch.cuda.synchronize()
-        assert torch.equal(mk, a[:size]) and torch.equal(mv, pa[:size]), f"pairs n={size}"
-        assert reflib.lib.ref_validate_keys(h, mk.data_ptr(), size) == 0  # the reference's own validator on OUR output
-    reflib.lib.ref_destroy(h)
+        assert device_digest(mk) == want["sorted_digest"] and device_digest(mv) == want["payload_digest"], f"pairs n={size}"
 
 
 @pytest.mark.skipif(not os.path.exists(GOLDEN), reason="golden fixture not generated yet")

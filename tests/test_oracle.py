@@ -107,3 +107,20 @@ def test_oracle_reproduces_reference_golden_vectors(oracle):
         assert [int(x) for x in sk[-8:]] == c["sorted_tail"]
         assert oracle.digest(sk) == c["sorted_digest"]
         assert oracle.digest(oracle.global_histogram(k).reshape(-1)) == c["global_hist_digest"]
+
+
+def test_oracle_reproduces_reference_parity_digests(oracle):
+    """The device digests the reference produced for the GPU parity tests (tests/golden/make_ref_golden.py), recomputed
+    on the CPU from the oracle: pins the fixture and oraclelib.device_digest, whatever device it runs on."""
+    import torch
+
+    from tests.oraclelib import device_digest
+
+    cases = json.load(open(os.path.join(os.path.dirname(GOLDEN), "ref_onesweep_parity_golden.json")))["bit_exact"]
+    assert len(cases) == 4
+    for c in cases:
+        k = oracle.init_random_u32(c["n"], 0, c["seed"])
+        sk, sv = oracle.sort_pairs(k, k.copy())
+        assert device_digest(torch.from_numpy(k.view(np.int32))) == c["keys"]["input_digest"] == c["pairs"]["input_digest"]
+        assert device_digest(torch.from_numpy(sk.view(np.int32))) == c["keys"]["sorted_digest"] == c["pairs"]["sorted_digest"]
+        assert device_digest(torch.from_numpy(sv.view(np.int32))) == c["pairs"]["payload_digest"]
