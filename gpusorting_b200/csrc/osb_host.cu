@@ -136,6 +136,9 @@ int sort_impl(osb200_sorter* s, void* d_keys, uint32_t* d_vals, uint64_t n, cuda
     if (!d_keys || (reinterpret_cast<uintptr_t>(d_keys) & 15u)) return OSB200_ERR_INVALID_ARG;
     // d_vals == nullptr is a keys-only sort (also on a pairs-capable handle); the handle is never modified to say so
     if (d_vals && !s->value_bytes) return OSB200_ERR_INVALID_ARG;
+    // payloads need the keys' 16-byte alignment: the copy-back after an odd number of executed passes moves them as uint4.
+    // Checked for every n, so that whether a call is accepted does not depend on which path its size takes.
+    if (reinterpret_cast<uintptr_t>(d_vals) & 15u) return OSB200_ERR_INVALID_ARG;
     const int places = (end_bit - begin_bit + 7) / 8;
     const uint32_t last_bits = static_cast<uint32_t>(end_bit - begin_bit - 8 * (places - 1));
     const bool whole_key = begin_bit == 0 && end_bit == key_bits;

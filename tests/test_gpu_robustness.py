@@ -156,6 +156,33 @@ def test_sort_bits_rejects_bad_ranges(g, sorter):
             sorter.sort_bits(t, b, e)
 
 
+@pytest.mark.parametrize("n", [5000, 16384 * 3 + 77])
+def test_misaligned_payloads_are_rejected(g, sorter, n):
+    """Payloads must be 16-byte aligned like the keys: after an odd number of executed passes the copy-back moves them
+    in 16-byte words.  Keys below 2^24 skip the top byte's pass (3 executed) -- the case a misaligned payload would fault
+    in -- and the small-n path (n = 5000) refuses it too, so acceptance does not depend on n.  A refused call leaves both
+    buffers untouched, and the handle sorts correctly afterwards."""
+    k = (np.random.default_rng(n).integers(0, 1 << 24, n)).astype(np.uint32)
+    tk = dev(k)
+    storage = torch.arange(n + 1, dtype=torch.int32, device="cuda")
+    tv = storage[1:]  # contiguous, 4-byte aligned only
+    assert tv.data_ptr() % 16 == 4
+    v0 = tv.clone()
+    calls = [lambda: sorter.sort_pairs(tk, tv), lambda: sorter.sort_bits(tk, 0, 24, tv),
+             lambda: sorter.sort_pairs_typed(tk, tv, "i32", True)]
+    for call in calls:
+        with pytest.raises(g.OneSweepError) as e:
+            call()
+        assert e.value.status == -1
+        assert np.array_equal(host(tk), k) and torch.equal(tv, v0), "a refused sort must not touch the buffers"
+    tv = torch.arange(n, dtype=torch.int32, device="cuda")
+    sorter.sort_pairs(tk, tv)
+    order = np.argsort(k, kind="stable")
+    assert np.array_equal(host(tk), k[order]) and np.array_equal(host(tv), order.astype(np.uint32))
+    if n > sorter.info("small_path_max_n"):
+        assert sorter.info("last_skip_mask") == 0b1000 and sorter.info("last_executed_passes") == 3
+
+
 @pytest.mark.parametrize("stall_every", [1, 2, 5])
 def test_lookback_fallback_rereduces_stalled_tiles(g, oracle, stall_every):
     """Forward-progress fallback (EmulatedDeadlocking.cu:159-267; test hook as :339-345): every N-th tile WITHHOLDS its

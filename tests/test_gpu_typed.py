@@ -1,26 +1,15 @@
 """Typed keys and descending order (SURVEY 8f rank 1): the order-preserving bit transforms of the reference's HLSL path
 (GPUSortingD3D12/Shaders/SortCommon.hlsl:134-154 FloatToUint / IntToUint, :594-656 descending) fused into the first
 and last OneSweep pass.  Oracle: numpy restatement of those transforms + a stable argsort.  -m gpu"""
+import zlib
+
 import numpy as np
 import pytest
 import torch
 
+from tests.sortcheck import radix_key as to_radix
+
 pytestmark = pytest.mark.gpu
-
-
-def to_radix(bits: np.ndarray, kind: str, descending: bool) -> np.ndarray:
-    """unsigned key whose ascending order is the requested order of the typed value (reference transform)"""
-    nb = bits.dtype.itemsize * 8
-    u = bits.copy()
-    sign = np.array(1 << (nb - 1), dtype=bits.dtype)
-    if kind == "i":
-        u ^= sign
-    elif kind == "f":
-        neg = (u >> np.array(nb - 1, dtype=bits.dtype)).astype(bool)
-        u = np.where(neg, ~u, u | sign)
-    if descending:
-        u = ~u
-    return u
 
 
 CASES = [("u32", np.uint32, "u"), ("i32", np.uint32, "i"), ("f32", np.uint32, "f"),
@@ -44,7 +33,7 @@ def make_bits(rng, n, dtype, kind):
 def test_typed_keys(name, dtype, kind, descending):
     import gpusorting_b200 as g
 
-    rng = np.random.default_rng(hash(name) & 0xFFFF)
+    rng = np.random.default_rng(zlib.crc32(name.encode()) & 0xFFFF)  # the same seed in every process
     kb = np.dtype(dtype).itemsize
     s = g.OneSweepSorter(1 << 20, kb, 0)
     T = s.info("tile_keys")
